@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torch.distributed.run, one rank per GPU)
   python bench.py --impl reference --steps K --warmup W     (the reference's own CPU train_one_epoch on the host cores)
+  python bench.py --steps K --warmup W --dump-outputs DIR   (also writes what the last timed step computed, as .npy files)
 
 One step = forward + soft-max cross-entropy + backward + gradient all-reduce + SGD(momentum) update, i.e. the body of the
 reference's train_one_epoch (classification/resnet/utils.py:35-55) in the DDP pattern of others/train_with_DDP.
@@ -255,6 +256,23 @@ def optimizer_desc(name):
             "AdamW(lr=5e-4, wd=5e-2, decay groups)" if name in ADAMW_MODELS else "SGD(momentum=0.9, weight_decay=5e-5)")
 
 
+DUMP_PARAM_SAMPLE = 1 << 20   # parameters per model written by --dump-outputs (4 MB in fp32)
+
+
+def dump_outputs(out_dir, name, loss, correct, flat_p):
+    """What the last timed step returned (loss, per-sample correct flags) and a fixed, seeded sample of the parameters it
+    updated, as float32 DIR/<model>_<array>.npy: two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = flat_p.numel()
+    idx = torch.randint(0, n, (min(n, DUMP_PARAM_SAMPLE),), generator=torch.Generator().manual_seed(0)).unique()
+    arrays = {"loss": loss, "correct": correct, "params_sample": flat_p[idx.to(flat_p.device)]}
+    for key, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}_{key}.npy"), t.detach().float().cpu().numpy())
+
+
 def measure(name, args, dev, world, rank, local_rank, batch=None):
     """All measurements of one model: device-resident throughput, e2e, per-kernel spans.  Returns the JSON dict (every rank
     runs everything; only rank 0's dict carries the roofline / kernel table)."""
@@ -306,7 +324,7 @@ def measure(name, args, dev, world, rank, local_rank, batch=None):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        loss, _ = trainer.step(images, labels)
+        loss, correct = trainer.step(images, labels)
     e1.record()
     sync_all()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
@@ -315,6 +333,8 @@ def measure(name, args, dev, world, rank, local_rank, batch=None):
     final_loss = float(loss)
     ms_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, name, loss, correct, trainer.arena.flat_p)
 
     # ---- end-to-end: pinned host batch -> H2D every step (double-buffered on a copy stream), loss read back ---------
     host_imgs = [torch.randn(B, 3, 224, 224).pin_memory() for _ in range(2)]
@@ -504,7 +524,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the ViT-B/16 block of the default (resnet50) line")
     ap.add_argument("--eager", action="store_true", help="do not capture the step into CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the last step's loss, correct flags and a seeded sample of the updated "
+                         "parameters of each measured model to DIR/<model>_<array>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 training step (--impl b200)")
     global _JSON_FD
     sys.stdout.flush()
     _JSON_FD = os.dup(1)

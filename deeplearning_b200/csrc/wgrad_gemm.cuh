@@ -67,7 +67,6 @@ __global__ void __launch_bounds__(kBias ? 320 : 192, 1) wgrad_gemm_kernel(const 
   uint64_t* tmem_full = bars + 2 * STAGES;
   uint64_t* tmem_empty = bars + 2 * STAGES + 2;
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(bars + 2 * STAGES + 4);
-  uint64_t* item_bar = bars + 2 * STAGES + 5;   // kBias: the MMA thread has reached the next item the column-sum warps read
 
   const int warp_idx = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
@@ -80,13 +79,12 @@ __global__ void __launch_bounds__(kBias ? 320 : 192, 1) wgrad_gemm_kernel(const 
     for (int i = 0; i < 4; ++i) tma_prefetch_desc(&p.x_maps[i]);
     for (int i = 0; i < STAGES; ++i) {
       mbar_init(&full_bar[i], 1);
-      mbar_init(&empty_bar[i], kBias ? 5 : 1);   // the MMA commit (+ the four column-sum warps)
+      mbar_init(&empty_bar[i], kBias ? 5 : 1);   // the MMA commit (+ the four column-sum warps, on every stage)
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tmem_full[i], 1);
       mbar_init(&tmem_empty[i], 4);
     }
-    mbar_init(item_bar, 1);
     fence_mbar_init();
   }
   if (warp_idx == 1) tmem_alloc<Cfg::TMEM_COLS>(tmem_ptr_smem);
@@ -159,30 +157,12 @@ __global__ void __launch_bounds__(kBias ? 320 : 192, 1) wgrad_gemm_kernel(const 
         const int split = item / items_per_split;
         const int kb0 = split * p.kb_per_split;
         const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
-        bool summed = false;   // kBias: is this the item whose dY tiles the column-sum warps read?
-        if constexpr (kBias) {
-          int r = item - split * items_per_split;
-          const int tap = r % p.num_taps;
-          r /= p.num_taps;
-          summed = (r % p.ng_tiles) == 0 && tap == 0;
-        }
         mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
         tc_fence_after();
-        if constexpr (kBias) {
-          // every earlier tile has been consumed: the column-sum warps may now start waiting for this item's tiles (an
-          // mbarrier parity wait is only meaningful for a waiter that is less than one phase ahead of the pipeline)
-          if (summed) mbar_arrive(item_bar);
-        }
         const uint32_t tmem_d = tmem_base + acc * BLOCK_NG;
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
-          if constexpr (kBias) {
-            if (!summed) {   // nobody else reads this tile: stand in for the four column-sum warps
-#pragma unroll
-              for (int i = 0; i < 4; ++i) mbar_arrive(&empty_bar[stage]);
-            }
-          }
           // 16 pixel rows per MMA = 2048 B; LBO = next 64-channel atom (8192 B); SBO = next 8 pixel rows (1024 B)
           const uint64_t soff = static_cast<uint64_t>(stage) * (Cfg::STAGE_BYTES >> 4);
           const uint64_t da = desc_a0 + soff, db = desc_b0 + soff;
@@ -204,8 +184,9 @@ __global__ void __launch_bounds__(kBias ? 320 : 192, 1) wgrad_gemm_kernel(const 
     }
   } else if (kBias && warp_idx >= 6) {
     // ===================== column sums of the dY tiles (bias gradient) =====================
-    // Only the (ng == 0, tap == 0) item of every (split, mg) pair is summed; for all other items the MMA thread supplies
-    // this role's four arrivals itself (below), so the pipeline of those items is untouched.
+    // Only the (ng == 0, tap == 0) item of every (split, mg) pair is summed, but these warps wait for and release every stage
+    // of every item, in order, like any other consumer of the ring: a CTA that runs several items (more items than SMs)
+    // keeps its phase bookkeeping exact, and no tile is refilled before they are done with it.
     // The dY stage is 64 pixel rows x 2 atoms x 128 B: thread t of the 128 reads 8 rows of ONE 16-byte chunk (8 channels),
     // chunk cc = t % 16 (atom cc / 8, chunk cc % 8 inside the 128-byte row, XOR-swizzled by row & 7), rows (t / 16) * 8 .. + 8.
     __shared__ float bias_red[8][128];
@@ -213,7 +194,7 @@ __global__ void __launch_bounds__(kBias ? 320 : 192, 1) wgrad_gemm_kernel(const 
     const int cc = t & 15, rg = t >> 4;
     const uint32_t atom_off = static_cast<uint32_t>(cc >> 3) * 8192u;
     int stage = 0;
-    uint32_t phase = 0, item_phase = 0;
+    uint32_t phase = 0;
     for (int item = blockIdx.x; item < num_items; item += gridDim.x) {
       const int split = item / items_per_split;
       int r = item - split * items_per_split;
@@ -223,40 +204,38 @@ __global__ void __launch_bounds__(kBias ? 320 : 192, 1) wgrad_gemm_kernel(const 
       const int mg = r / p.ng_tiles;
       const int kb0 = split * p.kb_per_split;
       const int kb1 = min(p.kb_total, kb0 + p.kb_per_split);
-      if (!(ng == 0 && tap == 0)) {
-        // not ours: just keep the ring position in step
-        const int n = kb1 - kb0;
-        const int adv = stage + n;
-        phase ^= static_cast<uint32_t>((adv / STAGES) & 1);
-        stage = adv % STAGES;
-        continue;
-      }
+      const bool summed = ng == 0 && tap == 0;
       float sum[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      mbar_wait(item_bar, item_phase);   // the pipeline has reached this item
-      item_phase ^= 1;
       for (int kb = kb0; kb < kb1; ++kb) {
         mbar_wait(&full_bar[stage], phase);
-        const uint32_t base = smem_u32(smem + stage * Cfg::STAGE_BYTES) + atom_off;
-        uint4 v[8];
+        if (summed) {
+          const uint32_t base = smem_u32(smem + stage * Cfg::STAGE_BYTES) + atom_off;
+          uint4 v[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const int row = rg * 8 + i;
-          v[i] = lds128(base + row * 128 + ((static_cast<uint32_t>(cc & 7) ^ static_cast<uint32_t>(row & 7)) << 4));
+          for (int i = 0; i < 8; ++i) {
+            const int row = rg * 8 + i;
+            v[i] = lds128(base + row * 128 + ((static_cast<uint32_t>(cc & 7) ^ static_cast<uint32_t>(row & 7)) << 4));
+          }
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            float f[8];
+            unpack8(v[i], f);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) sum[j] += f[j];
+          }
+          // the sums depend on every word loaded from the tile: computing them here means the loads have returned before
+          // the release below lets the producer overwrite the stage
+          asm volatile("" ::"f"(sum[0]), "f"(sum[1]), "f"(sum[2]), "f"(sum[3]), "f"(sum[4]), "f"(sum[5]), "f"(sum[6]),
+                       "f"(sum[7]) : "memory");
         }
         __syncwarp();
-        if (lane == 0) mbar_arrive(&empty_bar[stage]);   // the tile has been read
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          float f[8];
-          unpack8(v[i], f);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) sum[j] += f[j];
-        }
+        if (lane == 0) mbar_arrive(&empty_bar[stage]);   // this warp is done with the tile
         if (++stage == STAGES) {
           stage = 0;
           phase ^= 1;
         }
       }
+      if (!summed) continue;
       // fold the 8 row groups (fixed order: deterministic) and write this split's partial sums
       named_bar_sync(2, 128);   // previous item's readers are done with bias_red
 #pragma unroll

@@ -27,3 +27,46 @@ class CpuSgdTrainer:
         self.opt.step()
         self.opt.zero_grad()
         return float(loss.detach()), correct
+
+
+def train_one_epoch(model, data_loader, device, optimizer, loss_function):
+    """The reference's ``train_one_epoch`` protocol (classification/resnet/utils.py:28-57) on any module, without its
+    per-step prints: the loss is summed in an fp32 tensor on ``device``.  Returns (mean loss per step, accuracy over the
+    samples seen), as the reference does.  ``tests/golden/make_golden.py`` checks that this loop and ``evaluate`` return
+    exactly what the reference's own loops return; ``tests/golden/resnet50_loops.json`` keeps those values."""
+    model.train()
+    loss_sum = torch.zeros(1, device=device)
+    correct = torch.zeros(1, device=device)
+    optimizer.zero_grad()
+    seen = steps = 0
+    for images, labels in data_loader:
+        images, labels = images.to(device), labels.to(device)
+        seen += images.shape[0]
+        steps += 1
+        pred = model(images)
+        correct += (pred.argmax(1) == labels).sum()
+        loss = loss_function(pred, labels)
+        loss.backward()
+        loss_sum += loss.detach()
+        if not torch.isfinite(loss):
+            raise FloatingPointError(f"non-finite training loss {float(loss)}")
+        optimizer.step()
+        optimizer.zero_grad()
+    return loss_sum.item() / steps, correct.item() / seen
+
+
+@torch.no_grad()
+def evaluate(model, data_loader, device, loss_function):
+    """The reference's ``evaluate`` protocol (classification/resnet/utils.py:60-83): eval mode, no autograd, same return."""
+    model.eval()
+    loss_sum = torch.zeros(1, device=device)
+    correct = torch.zeros(1, device=device)
+    seen = steps = 0
+    for images, labels in data_loader:
+        images, labels = images.to(device), labels.to(device)
+        seen += images.shape[0]
+        steps += 1
+        pred = model(images)
+        correct += (pred.argmax(1) == labels).sum()
+        loss_sum += loss_function(pred, labels)
+    return loss_sum.item() / steps, correct.item() / seen

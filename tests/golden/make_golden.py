@@ -7,6 +7,7 @@ of deeplearning_b200 produces a bit-identical state_dict under the same seed, (3
 bit-identical logits / loss / gradients / buffer updates on the same weights and input, and (4) stores small outputs.
 """
 import importlib.util
+import json
 import os
 import sys
 import types
@@ -327,17 +328,66 @@ def droppath_fixture():
     return out
 
 
+def resnet50_loops_fixture():
+    """The reference's own ``evaluate`` and ``train_one_epoch`` (classification/resnet/utils.py) on its resnet50(), CPU fp32,
+    with the running statistics calibrated on one batch first: their return values, and the check that the restated loops
+    of oracle/train_loop.py return the same numbers bit for bit."""
+    from oracle.resnet import resnet_forward
+    from oracle.train_loop import evaluate, train_one_epoch
+
+    _shim("matplotlib")
+    _shim("matplotlib.pyplot")
+    utils = _load(f"{REF}/classification/resnet/utils.py", "ref_resnet_utils")
+    ref_mod = _load(f"{REF}/classification/resnet/models/networks.py", "ref_resnet_networks_loops")
+    seeds = {"init": 0, "calib": 3, "batches": 5}
+    torch.manual_seed(seeds["init"])
+    state = {k: v.clone() for k, v in ref_mod.resnet50().state_dict().items()}
+    xc = torch.randn(32, 3, 224, 224, generator=torch.Generator().manual_seed(seeds["calib"]))
+    with torch.no_grad():
+        resnet_forward(state, xc, train=True, momentum=1.0)
+    g = torch.Generator().manual_seed(seeds["batches"])
+    batches = [(torch.randn(8, 3, 224, 224, generator=g), torch.randint(0, 1000, (8,), generator=g)) for _ in range(2)]
+    cpu, loss_fn = torch.device("cpu"), torch.nn.CrossEntropyLoss()
+    out = {"seeds": seeds, "calib_batch": 32, "batch": 8, "steps": 2, "lr": 0.01, "momentum": 0.9, "weight_decay": 5e-5}
+    loops = {"reference": (lambda m: utils.evaluate(m, batches, cpu, loss_fn, 0),
+                           lambda m, opt: utils.train_one_epoch(m, batches, cpu, opt, loss_fn, 0)),
+             "oracle": (lambda m: evaluate(m, batches, cpu, loss_fn),
+                        lambda m, opt: train_one_epoch(m, batches, cpu, opt, loss_fn))}
+    for which, (ev, tr) in loops.items():
+        model = ref_mod.resnet50()
+        model.load_state_dict(state)
+        e = ev(model)
+        opt = torch.optim.SGD(model.parameters(), lr=out["lr"], momentum=out["momentum"], weight_decay=out["weight_decay"])
+        t = tr(model, opt)
+        res = {"eval_loss": e[0], "eval_acc": e[1], "train_loss": t[0], "train_acc": t[1],
+               "fc_weight_norm_after": float(model.fc.weight.detach().double().norm())}
+        if which == "reference":
+            out.update(res)
+        else:
+            assert res == {k: out[k] for k in res}, ("oracle loops differ from the reference's", res)
+    return out
+
+
 FIXTURES = {"resnet50": resnet50_fixture, "mnist": mnist_fixture, "vit_b16": vit_fixture, "convnext_tiny": convnext_fixture,
             "swin_tiny": swin_fixture, "droppath": droppath_fixture}
+# plain numbers, kept in a JSON file of their own: {name: (fixture, file name)}
+JSON_FIXTURES = {"resnet50_loops": (resnet50_loops_fixture, "resnet50_loops.json")}
 
 if __name__ == "__main__":
     torch.set_num_threads(8)
-    path = os.path.join(HERE, "classification_golden.pt")
     only = sys.argv[1:]   # e.g. `make_golden.py swin_tiny` refreshes one entry and keeps the others
-    fx = torch.load(path, weights_only=False) if only else {}
-    for name, fn in FIXTURES.items():
+    for name, (fn, fname) in JSON_FIXTURES.items():
         if not only or name in only:
-            fx[name] = fn()
-    fx["torch"] = torch.__version__
-    torch.save(fx, path)
-    print("golden fixtures written:", os.path.join(HERE, "classification_golden.pt"), os.path.getsize(os.path.join(HERE, "classification_golden.pt")), "bytes")
+            with open(os.path.join(HERE, fname), "w") as f:
+                json.dump(fn(), f, indent=1)
+                f.write("\n")
+            print("golden fixture written:", os.path.join(HERE, fname))
+    if not only or set(only) & set(FIXTURES):
+        path = os.path.join(HERE, "classification_golden.pt")
+        fx = torch.load(path, weights_only=False) if only else {}
+        for name, fn in FIXTURES.items():
+            if not only or name in only:
+                fx[name] = fn()
+        fx["torch"] = torch.__version__
+        torch.save(fx, path)
+        print("golden fixtures written:", path, os.path.getsize(path), "bytes")

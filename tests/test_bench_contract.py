@@ -53,3 +53,24 @@ def test_b200_arm_fails_loudly_without_gpu():
     assert r.returncode != 0
     assert r.stdout.strip() == ""          # no JSON line from a fallback path
     assert "no CUDA device" in r.stderr or "CUDA" in r.stderr
+
+
+def test_dump_outputs_writes_a_fixed_float32_sample(tmp_path):
+    """--dump-outputs: float32 .npy files, the same parameter sample on every call, its size capped whatever the model."""
+    import numpy as np
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    flat_p = torch.randn(3 * bench.DUMP_PARAM_SAMPLE)
+    loss, correct = torch.tensor([6.9]), torch.tensor([0, 1, 1, 0], dtype=torch.int32)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), "m", loss, correct, flat_p)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == ["m_correct.npy", "m_loss.npy", "m_params_sample.npy"]
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float32 and np.array_equal(a, b), n
+    sample = np.load(tmp_path / "a" / "m_params_sample.npy")
+    assert 0 < sample.size <= bench.DUMP_PARAM_SAMPLE and np.isin(sample, flat_p.numpy()).all()
+    assert np.array_equal(np.load(tmp_path / "a" / "m_correct.npy"), [0, 1, 1, 0])

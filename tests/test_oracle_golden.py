@@ -3,6 +3,7 @@
 The weights are re-created by the host-side mirror constructors under the recorded seed, so these tests pin three things at
 once without /root/reference: constructor init == reference init, oracle forward/backward == reference, fixtures unchanged.
 """
+import json
 import os
 
 import pytest
@@ -190,3 +191,48 @@ def test_droppath_oracle_matches_reference(name):
     for n, g in grads.items():
         ref = fx[name]["grad_norms"][n]
         assert abs(float(g.double().norm()) - ref) <= 2e-3 * (ref + 1e-6), n
+
+
+class _OracleResNet(torch.nn.Module):
+    """The fp32 oracle ResNet as a module: parameters registered for an optimizer, running statistics updated in place."""
+
+    def __init__(self, state):
+        super().__init__()
+        self.state = dict(state)
+        self.params = torch.nn.ParameterList()
+        for k, v in state.items():
+            if v.is_floating_point() and "running_" not in k:
+                self.state[k] = torch.nn.Parameter(v.clone())
+                self.params.append(self.state[k])
+
+    def forward(self, x):
+        from oracle.resnet import resnet_forward
+
+        return resnet_forward(self.state, x, train=self.training)
+
+
+def test_resnet50_epoch_loops_match_reference():
+    """oracle/train_loop.py's evaluate / train_one_epoch (the loops tests/test_gpu_resnet.py drives the drop-in module with)
+    return what the reference's own loops returned on the same weights and batches (make_golden.py, there bit for bit)."""
+    from deeplearning_b200.classification.resnet.models.networks import resnet50
+    from oracle.resnet import resnet_forward
+    from oracle.train_loop import evaluate, train_one_epoch
+
+    with open(os.path.join(HERE, "golden", "resnet50_loops.json")) as f:
+        fx = json.load(f)
+    torch.manual_seed(fx["seeds"]["init"])
+    state = {k: v.clone() for k, v in resnet50().state_dict().items()}
+    xc = torch.randn(fx["calib_batch"], 3, 224, 224, generator=torch.Generator().manual_seed(fx["seeds"]["calib"]))
+    with torch.no_grad():
+        resnet_forward(state, xc, train=True, momentum=1.0)
+    g = torch.Generator().manual_seed(fx["seeds"]["batches"])
+    batches = [(torch.randn(fx["batch"], 3, 224, 224, generator=g), torch.randint(0, 1000, (fx["batch"],), generator=g))
+               for _ in range(fx["steps"])]
+    model, cpu, loss_fn = _OracleResNet(state), torch.device("cpu"), torch.nn.CrossEntropyLoss()
+    loss, acc = evaluate(model, batches, cpu, loss_fn)
+    assert abs(loss - fx["eval_loss"]) < 1e-4 and acc == fx["eval_acc"], (loss, acc)
+    opt = torch.optim.SGD(model.parameters(), lr=fx["lr"], momentum=fx["momentum"], weight_decay=fx["weight_decay"])
+    loss, acc = train_one_epoch(model, batches, cpu, opt, loss_fn)
+    assert abs(loss - fx["train_loss"]) < 1e-4 and acc == fx["train_acc"], (loss, acc)
+    norm = float(model.state["fc.weight"].detach().double().norm())
+    assert abs(norm - fx["fc_weight_norm_after"]) <= 1e-5 * fx["fc_weight_norm_after"], norm
